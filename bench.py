@@ -2,13 +2,14 @@
 """OSVOS hot-path benchmark (contract: the task statement; method: DESIGN.md section 6).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload infer480|train480|parent480]
+                    [--dump-outputs DIR]
 
 Default run (`--workload infer480`, what the driver launches), ONE JSON line on rank 0:
 
   headline   BASELINE.json configs[1]: forward of one 480x854 frame per step and GPU, device-resident (`value`) and end to
-             end from pinned host memory (`e2e`).  One timed BLOCK = exactly K steps between barrier + synchronize pairs,
-             CUDA events on the launching stream, max over ranks.  K steps of a 0.7 ms frame are too short a window to
-             trust, so blocks are repeated until >= 1 s has been timed and the MEDIAN block is reported (`blocks`).
+             end from pinned host memory (`e2e`).  Each is timed over exactly K steps between barrier + synchronize
+             pairs, CUDA events on the launching stream, max over ranks.  K steps of a 0.7 ms frame are a short window:
+             it takes a K of about 1500 to time a second.
   dp         BASELINE.json configs[3], the one multi-GPU path north_star names: parent training, batch 12 per GPU at
              480x854, 5-loss objective, FusedSGD, ONE NCCL allreduce(mean) of the 59.7 MB gradient bucket per step; run
              at every N including 1, with its own parity check (R ranks x 1 small frame against the oracle's
@@ -21,6 +22,12 @@ Default run (`--workload infer480`, what the driver launches), ONE JSON line on 
   cpu_baseline    the same reference modules on the host cores (bounded sample).
 
 `--impl reference` times the reference's own CPU path (oracle/_ref when present, else the oracle port).
+
+`--dump-outputs DIR` writes what the timed path returned in its last step as DIR/<name>.npy (float32): the five logit
+maps (infer480), the loss and the parameter gradients of that step (train480), the five losses and the updated
+parameters (parent480).  Inputs and weights are seeded, so two builds run with the same arguments can be compared
+output for output: the inference maps bit for bit; the training paths with a tolerance, as their gradient reductions are
+not deterministic.
 """
 import argparse
 import json
@@ -48,8 +55,7 @@ sys.path.insert(0, ROOT)
 
 H, W = 480, 854
 METRIC = "frames/sec at 480x854 fwd-only, batch 1 per GPU (OSVOS.forward -> 5 logit maps)"
-MIN_TIMED_MS = 1000.0          # blocks of K steps are repeated until this much has been timed
-MAX_BLOCKS = 400
+MAX_DUMP_BYTES = 64 * 10**6    # --dump-outputs budget
 
 
 def workload_label(workload):
@@ -276,16 +282,21 @@ class Timer:
         self.barrier()
         return self.max_over_ranks(e0.elapsed_time(e1))
 
-    def blocks(self, fn, k, after=None, min_ms=MIN_TIMED_MS, min_blocks=3):
-        """Repeat the k-step block until >= min_ms has been timed (same count on every rank: derived from the first,
-        already rank-maximised block).  -> (median ms per step, info dict)."""
-        first = self.block(fn, k, after)
-        n = int(min(MAX_BLOCKS, max(min_blocks, math.ceil(min_ms / max(first, 1e-3)))))
-        times = [first] + [self.block(fn, k, after) for _ in range(n - 1)]
-        med = statistics.median(times)
-        return med / k, {"blocks": len(times), "steps_per_block": k, "timed_ms_total": sum(times),
-                         "ms_per_step_median": med / k, "ms_per_step_min": min(times) / k, "ms_per_step_max": max(times) / k,
-                         "reported": "median block"}
+    def steps(self, fn, k, after=None):
+        """Exactly k timed steps in one block -> (ms per step, info dict)."""
+        ms = self.block(fn, k, after)
+        return ms / k, {"timed_steps": k, "timed_ms_total": ms}
+
+
+def dump_outputs(out_dir, arrays):
+    """{name: tensor} -> out_dir/<name>.npy in float32."""
+    import numpy as np
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= MAX_DUMP_BYTES, f"--dump-outputs: {total} bytes exceed {MAX_DUMP_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -331,8 +342,9 @@ def dp_parity(rank, world, dev, precision):
             "ok": bool(max(head.values()) < tol_head and max(trunk.values()) < tol_trunk), "params_checked": len(errs)}
 
 
-def run_dp(args, rank, world, local, dev, timer, steps):
-    """-> the `dp` object (rank 0) : parent480, per-GPU batch `args.batch`, one allreduce(mean) + FusedSGD step per step."""
+def run_dp(args, rank, world, local, dev, timer, steps, dump_dir=None):
+    """-> the `dp` object (rank 0) : parent480, per-GPU batch `args.batch`, one allreduce(mean) + FusedSGD step per step.
+    dump_dir: rank 0 writes the last timed step's losses and the parameters it updated there."""
     import torch
     import torch.distributed as dist
     from osvos_pytorch_b200 import ops, parallel, training
@@ -364,7 +376,7 @@ def run_dp(args, rank, world, local, dev, timer, steps):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms, info = timer.blocks(one, steps, min_ms=MIN_TIMED_MS, min_blocks=2)
+    ms, info = timer.steps(one, steps)
     clocks = sampler.stop() if rank == 0 else None
     # the collective as it ran INSIDE the steps (device time between the events around it on this rank: payload +
     # waiting for the slowest rank), and alone, back to back (payload only)
@@ -389,6 +401,9 @@ def run_dp(args, rank, world, local, dev, timer, steps):
     first, last = loss_log[0].tolist(), loss_log[-1].tolist()     # device tensors until here: no host sync per step
     if rank != 0:
         return None
+    if dump_dir is not None:
+        dump_outputs(dump_dir, {"losses": loss_log[-1], **{"param." + n: p for n, p in net.named_parameters()
+                                                            if not n.startswith("upscale")}})
     fps = world * args.batch * 1000.0 / ms
     return {"workload": f"parent480 (BASELINE configs[3]): per-GPU batch {args.batch} x 3x{H}x{W} synthetic frames, global "
                         f"batch {world * args.batch}, 5-loss parent objective (train_parent.py:143-147), FusedSGD(lr {args.dp_lr:g}, "
@@ -510,14 +525,14 @@ def conv_traffic(precision, calls):
 def run_parent_headline(args, rank, world, local, dev, timer):
     """--workload parent480: the dp object promoted to the headline line."""
     import torch.distributed as dist
-    dp = run_dp(args, rank, world, local, dev, timer, max(1, args.steps))
+    dp = run_dp(args, rank, world, local, dev, timer, max(1, args.steps), args.dump_outputs)
     if rank == 0:
         emit({"metric": "frames/sec at 480x854 fwd+bwd, parent training (5-loss objective, SGD step, DP allreduce)",
               "value": dp["fps"], "unit": "frames/s", "n_gpus": world, "steps": dp["steps"], "warmup": 3,
               "ms_per_step": dp["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
               "dtype": dp["dtype"], "data": "synthetic",
               "config": {"workload": dp["workload"], "parallelism": dp["parallelism"],
-                         "l2": "per-step working set (>10 GB) exceeds L2", "timing": "CUDA events, max over ranks, median block"},
+                         "l2": "per-step working set (>10 GB) exceeds L2", "timing": "CUDA events over K steps, max over ranks"},
               "allreduce_ms": dp["allreduce_ms"], "allreduce_share": dp["allreduce_share"], "dp": dp,
               "gpu_launches": dp["gpu_launches"], "clocks": dp["clocks"]})
     if world > 1:
@@ -533,11 +548,13 @@ def main():
     ap.add_argument("--workload", default="infer480", choices=["infer480", "train480", "parent480"])
     ap.add_argument("--batch", type=int, default=12, help="parent480 / dp: frames per GPU per optimizer step")
     ap.add_argument("--precision", default="exact", choices=["exact", "fast"])
-    ap.add_argument("--dp-steps", type=int, default=10, help="optimizer steps per timed block of the dp leg")
+    ap.add_argument("--dp-steps", type=int, default=10, help="timed optimizer steps of the dp leg")
     ap.add_argument("--dp-lr", type=float, default=1e-10, help="learning rate of the dp leg (see run_dp)")
     ap.add_argument("--skip", default="", help="comma list of legs to skip: dp,parity,gpu_reference,cpu_baseline,roofline,e2e_extra")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--eager-train", action="store_true", help="train480: eager launches instead of the step graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step to "
+                                                          "DIR/<name>.npy (float32)")
     args = ap.parse_args()
     skip = {s for s in args.skip.split(",") if s}
     if args.no_cpu_baseline:
@@ -578,6 +595,7 @@ def main():
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
 
     graphed = {"step": None}
+    last = {}                                         # what the latest inference step returned
 
     def step(i, x=None):
         x = xs[i % n_in] if x is None else x
@@ -596,7 +614,8 @@ def main():
                     net, lambda outs, gt: class_balanced_cross_entropy_loss(outs[-1], gt, size_average=False), sample)
             return graphed["step"](sample)          # gradients accumulate, as between the reference's optimizer steps
         with torch.no_grad():
-            return net(x)[-1]
+            last["outs"] = net(x)
+        return last["outs"][-1]
 
     # kernels per step, counted on an eager pass (the timed inference steps replay a captured CUDA graph of
     # exactly these launches)
@@ -624,8 +643,18 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms, blocks_info = timer.blocks(step, steps)
+    ms, timed_info = timer.steps(step, steps)
     clocks = sampler.stop() if rank == 0 else None
+    dump = None
+    if args.dump_outputs is not None and rank == 0:
+        if train:
+            # the timed steps accumulate gradients: clear them and run the last timed step's frame once more
+            net.zero_grad(set_to_none=False)
+            dump = {"loss": step(steps - 1)}
+            dump.update(("grad." + n, p.grad) for n, p in net.named_parameters() if p.grad is not None)
+        else:
+            dump = {f"out{k}": o for k, o in enumerate(last["outs"])}
+        dump = {k: v.detach().cpu() for k, v in dump.items()}
 
     # ---- end to end: pinned host frame -> H2D -> OSVOS.forward -> D2H of the result ---
     def e2e_step(i):
@@ -639,31 +668,28 @@ def main():
     if train:
         for i in range(3):
             e2e_step(i)
-        ms_e2e, e2e_blocks = timer.blocks(e2e_step, steps)
+        ms_e2e, e2e_timed = timer.steps(e2e_step, steps)
     else:
         # the test-time loop of the reference (train_online.py:172-187) through the package's sequence pipeline:
         # every frame is copied H2D from pinned memory, run through OSVOS.forward, and its result copied D2H -
         # the three legs of consecutive frames overlap on separate streams (osvos_pytorch_b200/inference.py)
         from osvos_pytorch_b200.inference import SequenceSegmenter
 
-        def sequence_blocks(seg, k, **kw):
+        def sequence_timed(seg, k):
             for _ in seg(xs_host[i % n_in] for i in range(6)):      # warm-up, allocates the ring
                 pass
-            state = {}
 
-            def run_all(_i):                                          # one "step" of the block = the whole k-frame sequence
+            def run_all(_i):                                          # one timed "step" = the whole k-frame sequence
                 for _ in seg(xs_host[j % n_in] for j in range(k)):
                     pass
-            per_seq, info = timer.blocks(run_all, 1, after=seg.join_current_stream, **kw)
-            info = dict(info, steps_per_block=k, ms_per_step_median=info["ms_per_step_median"] / k,
-                        ms_per_step_min=info["ms_per_step_min"] / k, ms_per_step_max=info["ms_per_step_max"] / k)
-            return per_seq / k, info
-        ms_e2e, e2e_blocks = sequence_blocks(SequenceSegmenter(net, output="logits"), steps)
+            per_seq, info = timer.steps(run_all, 1, after=seg.join_current_stream)
+            return per_seq / k, dict(info, timed_steps=k)
+        ms_e2e, e2e_timed = sequence_timed(SequenceSegmenter(net, output="logits"), steps)
         if "e2e_extra" not in skip:
             for i in range(3):
                 e2e_step(i)
-            ms_serial, _ = timer.blocks(e2e_step, steps, min_ms=300.0)
-            ms_png, _ = sequence_blocks(SequenceSegmenter(net, output="bytescale"), steps, min_ms=300.0)
+            ms_serial, _ = timer.steps(e2e_step, steps)
+            ms_png, _ = sequence_timed(SequenceSegmenter(net, output="bytescale"), steps)
             e2e_extra = {"serial_single_stream": {"value": world * 1000.0 / ms_serial, "ms_per_step": ms_serial},
                          "u8_png_payload": {"value": world * 1000.0 / ms_png, "ms_per_step": ms_png,
                                             "d2h_bytes_per_step": H * W,
@@ -783,14 +809,13 @@ def main():
                                   f"parent-training path is the `dp` object of this line",
                    "l2": "per-step activation traffic (~0.9 GB exact) exceeds the 126 MB L2; inputs rotate over 4 frames; no explicit flush",
                    "timing": "CUDA events on the launching stream, max over ranks; W warm-up steps + 0.5 s of untimed steps, "
-                             "then blocks of exactly K steps (barrier + synchronize on both sides) repeated until >= 1 s "
-                             "is timed; the MEDIAN block is reported",
+                             "then exactly K timed steps (barrier + synchronize on both sides)",
                    "launch": ("captured CUDA graph of the step's kernels, replayed per step"
                               if ((graphs_on and not train) or (train and not args.eager_train)) else "eager launches")},
-        "blocks": blocks_info,
+        "timed": timed_info,
         "e2e": {"value": world * 1000.0 / ms_e2e, "unit": "frames/s", "ms_per_step": ms_e2e,
                 "h2d_bytes_per_step": 3 * H * W * 4, "d2h_bytes_per_step": (4 if train else H * W * 4),
-                "blocks": e2e_blocks,
+                "timed": e2e_timed,
                 "path": ("pinned host frame -> .to(cuda) -> fwd+loss+bwd -> D2H of the loss" if train else
                          "SequenceSegmenter: pinned host frame -> H2D -> OSVOS.forward (nn.Module API) -> D2H of the "
                          "fused logit map, legs of consecutive frames overlapped on 3 streams; the pipeline reads the fused "
@@ -851,6 +876,8 @@ def main():
                                 "sample": f"3 steps of the same 480x854 frame after 1 warm-up; "
                                           f"{'unmodified reference modules (oracle/_ref)' if kind == 'reference' else 'oracle port'}"
                                           f" = the reference's torch CPU fp32 path on {threads} threads ({cores} host cores)"}
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     emit(line)
 
 

@@ -6,7 +6,7 @@ import pytest
 import torch
 
 from oracle import osvos_oracle as oc
-from gpu_util import maxrel, rmsrel
+from gpu_util import golden_map, maxrel, rmsrel
 
 pytestmark = pytest.mark.gpu
 
@@ -22,10 +22,11 @@ def net():
     return m.cuda().eval()
 
 
-def mask_report(got, ref, tol):
-    got, ref = got.detach().cpu().numpy(), np.asarray(ref)
+def mask_report(got, ref, tol, scale=None):
+    got = got.detach().cpu().numpy() if isinstance(got, torch.Tensor) else np.asarray(got)
+    ref = np.asarray(ref)
     flips = (got > 0) != (ref > 0)
-    band = np.abs(ref) <= tol * np.abs(ref).max()
+    band = np.abs(ref) <= tol * (np.abs(ref).max() if scale is None else scale)
     inter = ((got > 0) & (ref > 0)).sum()
     union = ((got > 0) | (ref > 0)).sum()
     return int(flips.sum()), int((flips & ~band).sum()), float(inter / max(union, 1))
@@ -34,19 +35,27 @@ def mask_report(got, ref, tol):
 @pytest.mark.parametrize("tag,n,h,w,seed", [("fwd_48x70", 1, 48, 70, 11), ("fwd_33x45_n2", 2, 33, 45, 12),
                                             ("fwd_240x427", 1, 240, 427, 1234)])
 def test_forward_vs_reference_golden(net, golden, tag, n, h, w, seed):
+    """Of the 240x427 maps the fixture keeps a seeded sample of pixels: there the whole maps are also held to the
+    oracle, which tests/test_oracle.py pins to the reference."""
     x, _ = oc.synthetic_frame(n, h, w, seed)
     with torch.no_grad():
         outs = net(x.cuda())
     assert isinstance(outs, list) and len(outs) == 5
     for i, o in enumerate(outs):
-        ref = golden[f"{tag}.out{i}"]
         assert tuple(o.shape) == (n, 1, h, w) and o.dtype == torch.float32 and o.is_cuda
-        err = maxrel(o, ref)
-        flips, hard_flips, iou = mask_report(o, ref, LOGIT_TOL)
-        print(f"{tag} out{i}: maxrel {err:.2e} rmsrel {rmsrel(o, ref):.2e} flips {flips} (outside band {hard_flips}) IoU {iou:.6f}")
+        got, ref, scale = golden_map(golden, tag, i, o)
+        err = maxrel(got, ref, scale)
+        flips, hard_flips, iou = mask_report(got, ref, LOGIT_TOL, scale)
+        print(f"{tag} out{i}: maxrel {err:.2e} rmsrel {rmsrel(got, ref):.2e} flips {flips} (outside band {hard_flips}) IoU {iou:.6f}")
         assert err <= LOGIT_TOL
         assert hard_flips == 0
         assert iou > 0.999
+    if f"{tag}.idx" in golden:
+        with torch.no_grad():
+            full = oc.osvos_forward(oc.he_params(seed=0), x)
+        for i, (o, r) in enumerate(zip(outs, full)):
+            flips, hard_flips, iou = mask_report(o, r.numpy(), LOGIT_TOL)
+            assert maxrel(o, r) <= LOGIT_TOL and hard_flips == 0 and iou > 0.999, i
 
 
 def test_forward_stagewise_vs_oracle(net):

@@ -1,4 +1,7 @@
 """Drop-in surface of the OSVOS module (SURVEY.md section 8b) - CPU only, no compute."""
+import json
+import os
+
 import torch
 import torch.nn as nn
 
@@ -8,6 +11,7 @@ from osvos_pytorch_b200.networks.vgg_osvos import OSVOS
 
 import numpy as np
 import pytest
+import vgg_checkpoints
 
 
 @pytest.fixture(scope="module")
@@ -81,86 +85,49 @@ def test_layer_helpers(golden):
         L.class_balanced_cross_entropy_loss(torch.zeros(1, 1, 2, 2), torch.zeros(1, 1, 2, 2))
 
 
+def _reference_loaders():
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_loaders.json")) as f:
+        return json.load(f)
+
+
+def _assert_trunk_matches_reference(sd, ref):
+    assert list(sd.keys()) == ref["keys"]
+    got, want = vgg_checkpoints.trunk_digests(sd), ref["stages_sha256"]
+    assert len(want) == 26 and got.keys() == want.keys()
+    for name in want:
+        assert got[name] == want[name], name
+
+
 def test_caffe_vgg_loader_matches_the_reference_loader(tmp_path, monkeypatch):
     """`OSVOS(pretrained=2)` reads models/vgg_caffe.mat exactly like the reference's loader
     (networks/vgg_osvos.py:110-125): a synthetic .mat in the Caffe export layout (weights[0][k] = (kw, kh, cin, cout),
-    biases[0][k] = (cout, 1)) goes through BOTH loaders - the reference's own (oracle/_ref, unmodified) and this
-    package's - and every trunk tensor must come out bit-identical."""
-    import numpy as np
-    import scipy.io
-    import torch
-    from oracle import osvos_oracle as oc
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref not built (bash oracle/make_ref.sh; needs /root/reference)")
-    rng = np.random.default_rng(5)
-    shapes = [oc.param_shapes()[n + ".weight"] for n in oc.trunk_conv_names()]
-    weights = np.empty((1, len(shapes)), dtype=object)
-    biases = np.empty((1, len(shapes)), dtype=object)
-    for k, (co, ci, kh, kw) in enumerate(shapes):
-        weights[0, k] = rng.standard_normal((kw, kh, ci, co)).astype(np.float32)
-        biases[0, k] = rng.standard_normal((co, 1)).astype(np.float32)
+    biases[0][k] = (cout, 1)) goes through this package's loader, and every trunk tensor must come out bit-identical to
+    what the reference's own loader (unmodified) made of the same file (tests/golden/reference_loaders.json)."""
     (tmp_path / "models").mkdir()
-    scipy.io.savemat(str(tmp_path / "models" / "vgg_caffe.mat"), {"weights": weights, "biases": biases})
-    monkeypatch.chdir(tmp_path)                       # both Path.models_dir() default to ./models
+    weights = vgg_checkpoints.write_caffe_mat(str(tmp_path / "models" / "vgg_caffe.mat"))
+    monkeypatch.chdir(tmp_path)                       # Path.models_dir() defaults to ./models, as in the reference
     monkeypatch.delenv("OSVOS_MODELS_DIR", raising=False)
-    import contextlib
-    import io
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref_net = ref_loader.load().net.OSVOS(pretrained=2)
-    from osvos_pytorch_b200.networks.vgg_osvos import OSVOS
     mine = OSVOS(pretrained=2, verbose=False)
-    ref_sd, my_sd = ref_net.state_dict(), mine.state_dict()
-    assert list(ref_sd.keys()) == list(my_sd.keys())
-    checked = 0
-    for name in ref_sd:
-        if name.startswith("stages."):
-            assert torch.equal(ref_sd[name], my_sd[name]), name
-            checked += 1
-    assert checked == 26
+    my_sd = mine.state_dict()
+    _assert_trunk_matches_reference(my_sd, _reference_loaders()["caffe"])
     # the tensor the kernels will read is what Caffe stored: conv k, output channel o, input channel i, tap (r, s)
-    k, (co, ci, kh, kw) = 3, shapes[3]
+    k = 3
     w = my_sd[oc.trunk_conv_names()[k] + ".weight"]
     assert float(w[5, 7, 1, 2]) == float(weights[0, k][2, 1, 7, 5])
 
 
 def test_torchvision_vgg_loader_matches_the_reference_loader(tmp_path, monkeypatch):
     """`OSVOS(pretrained=1)` reads models/vgg_pytorch.pth like the reference's loader (networks/vgg_osvos.py:93-109): a
-    synthetic checkpoint of the reference's OWN `VGG` class (features + classifier, random weights) goes through both
-    loaders - the reference's (oracle/_ref, unmodified) and this package's - and every trunk tensor must be bit-identical."""
-    import contextlib
-    import io
-    import torch
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref not built (bash oracle/make_ref.sh; needs /root/reference)")
-    ref = ref_loader.load()
-    vgg_structure = [64, 64, 'M', 128, 128, 'M', 256, 256, 256, 'M', 512, 512, 512, 'M', 512, 512, 512, 'M']
-    torch.manual_seed(11)
-    vgg = ref.net.VGG(ref.net.make_layers(vgg_structure))
-    with torch.no_grad():
-        for m in vgg.features:
-            if isinstance(m, torch.nn.Conv2d):
-                m.weight.normal_(0.0, 0.05)
-                m.bias.normal_(0.0, 0.1)
+    synthetic checkpoint with the keys of torchvision's VGG-16 (features + classifier, random conv weights) goes through
+    this package's loader, and every trunk tensor must be bit-identical to what the reference's own loader (unmodified)
+    made of the same file (tests/golden/reference_loaders.json)."""
     (tmp_path / "models").mkdir()
-    torch.save(vgg.state_dict(), str(tmp_path / "models" / "vgg_pytorch.pth"))
-    want = [(m.weight.detach().clone(), m.bias.detach().clone()) for m in vgg.features if isinstance(m, torch.nn.Conv2d)]
-    del vgg
-    monkeypatch.chdir(tmp_path)                       # both Path.models_dir() default to ./models
+    want = vgg_checkpoints.write_torchvision_pth(str(tmp_path / "models" / "vgg_pytorch.pth"))
+    monkeypatch.chdir(tmp_path)                       # Path.models_dir() defaults to ./models, as in the reference
     monkeypatch.delenv("OSVOS_MODELS_DIR", raising=False)
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref_net = ref.net.OSVOS(pretrained=1)
-    from osvos_pytorch_b200.networks.vgg_osvos import OSVOS
     mine = OSVOS(pretrained=1, verbose=False)
-    ref_sd, my_sd = ref_net.state_dict(), mine.state_dict()
-    assert list(ref_sd.keys()) == list(my_sd.keys())
-    checked = 0
-    for name in ref_sd:
-        if name.startswith("stages."):
-            assert torch.equal(ref_sd[name], my_sd[name]), name
-            checked += 1
-    assert checked == 26
+    _assert_trunk_matches_reference(mine.state_dict(), _reference_loaders()["torchvision"])
     convs = [m for stage in mine.stages for m in stage if isinstance(m, torch.nn.Conv2d)]
+    assert len(convs) == len(want)
     for conv, (w, b) in zip(convs, want):
         assert torch.equal(conv.weight.detach(), w) and torch.equal(conv.bias.detach(), b)
