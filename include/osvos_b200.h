@@ -125,6 +125,25 @@ typedef struct {
 } osvos_conv3x3_args;
 OSVOS_API int osvos_conv3x3(const osvos_conv3x3_args* args /* host */, osvos_stream_t stream);
 
+/* ---- launch plans (tests / diagnosis) ----------------------------------------
+ * What osvos_conv3x3 / osvos_conv3x3_wgrad would launch for these arguments on the current device, under the
+ * current environment switches, without launching anything.  The launchers and the queries share one choice
+ * function, so the answer is the schedule the call runs.  The persistent kernels deal `items` work items round-robin
+ * to `grid` CTAs: CTA b runs items b, b + grid, b + 2 grid, ...                                                    */
+enum { OSVOS_TAP_ROWS = 3, OSVOS_TAP_PAIRS = 5, OSVOS_TAP_NINE = 9 };  /* wgrad tap items per (m, n) block */
+typedef struct {
+  int block_n;       /* output channels per tile (conv) / GEMM N per item (wgrad)                              */
+  int planes;        /* 2: exact split-bf16 operands, 1: FAST                                                    */
+  int split_acc;     /* 1: N-concatenated split accumulator (2 MMAs per K step instead of 3)                      */
+  int lean;          /* 1: the forward-only (lean) epilogue                                                     */
+  int items;         /* work items: output tiles (conv), (m block, n block, tap item, pixel split) items (wgrad) */
+  int grid;          /* CTAs launched                                                                          */
+  int tap_mode;      /* wgrad: OSVOS_TAP_*; 0 for conv                                                          */
+  int pixel_splits;  /* wgrad: pixel-range splits per tap item; 0 for conv                                      */
+} osvos_launch_plan;
+/* OSVOS_ERR_UNSUPPORTED when the arguments go to the side-branch kernel (cout == 2, or cout == 16 without act output). */
+OSVOS_API int osvos_conv3x3_plan(const osvos_conv3x3_args* args /* host */, osvos_launch_plan* plan /* host */);
+
 /* ---- folded side branch (inference and training) ---------------------------------------
  * side_prep has no ReLU (networks/vgg_osvos.py:67), so side_prep followed by score_dsn and this scale's slice of
  * fuse (:44,54,69,72) is ONE 3x3 convolution C -> 2:  W'[o][ci][tap] = sum_co proj_w[16 o + co] * side_w[co][ci][tap],
@@ -244,6 +263,8 @@ typedef struct {
 } osvos_wgrad_args;
 OSVOS_API size_t osvos_wgrad_workspace_bytes(int dz_channels, int cin);
 OSVOS_API int osvos_conv3x3_wgrad(const osvos_wgrad_args* args /* host */, osvos_stream_t stream);
+/* The launch plan of osvos_conv3x3_wgrad for these arguments (see osvos_conv3x3_plan). */
+OSVOS_API int osvos_conv3x3_wgrad_plan(const osvos_wgrad_args* args /* host */, osvos_launch_plan* plan /* host */);
 
 /* Deferred finish of up to OSVOS_WGRAD_FINISH_MAX weight gradients in ONE launch: workspace [9][a][b] -> OIHW,
  * dw = (accumulate ? dw : 0) + scale * ws.  With accumulate the destination can be the parameter's .grad itself

@@ -60,6 +60,15 @@ class WgradArgs(Structure):
                 ("dz_channels", c_int), ("flags", c_int)]
 
 
+class LaunchPlan(Structure):
+    """osvos_launch_plan (include/osvos_b200.h)."""
+    _fields_ = [("block_n", c_int), ("planes", c_int), ("split_acc", c_int), ("lean", c_int), ("items", c_int),
+                ("grid", c_int), ("tap_mode", c_int), ("pixel_splits", c_int)]
+
+
+TAP_ROWS, TAP_PAIRS, TAP_NINE = 3, 5, 9
+
+
 class WgradFinishItem(Structure):
     _fields_ = [("workspace", c_void_p), ("dw", c_void_p), ("cout", c_int), ("cin", c_int), ("dz_channels", c_int),
                 ("accumulate", c_int), ("scale", c_float)]
@@ -110,6 +119,7 @@ SIGNATURES = {
     "osvos_conv_first_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                      c_void_p]),
     "osvos_conv3x3": (c_int, [POINTER(Conv3x3Args), c_void_p]),
+    "osvos_conv3x3_plan": (c_int, [POINTER(Conv3x3Args), POINTER(LaunchPlan)]),
     "osvos_stage1_fused": (c_int, [POINTER(Stage1Args), c_void_p]),
     "osvos_set_pdl": (c_int, [c_int]),
     "osvos_fold_side_weights": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
@@ -122,6 +132,7 @@ SIGNATURES = {
     "osvos_cbce_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_double, c_size_t, c_void_p, c_void_p]),
     "osvos_wgrad_workspace_bytes": (c_size_t, [c_int, c_int]),
     "osvos_conv3x3_wgrad": (c_int, [POINTER(WgradArgs), c_void_p]),
+    "osvos_conv3x3_wgrad_plan": (c_int, [POINTER(WgradArgs), POINTER(LaunchPlan)]),
     "osvos_wgrad_finish": (c_int, [POINTER(WgradFinishItem), c_int, c_void_p]),
     "osvos_tail_bwd": (c_int, [POINTER(TailBwdArgs), c_void_p]),
     "osvos_tail_loss_bwd": (c_int, [POINTER(TailLossBwdArgs), c_void_p]),

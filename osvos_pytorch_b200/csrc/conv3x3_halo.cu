@@ -301,6 +301,9 @@ static HaloSwitches halo_switches() {
   return sw;
 }
 
+// persistent CTAs: one per tile up to one per SM; CTA b takes tiles b, b + grid, b + 2 grid, ...
+static int halo_grid(int tiles, int sms) { return tiles < sms ? tiles : sms; }
+
 template <int BLOCK_N, int PLANES, int PITCH, bool SPLIT = (PLANES == 2 && BLOCK_N <= 128), bool LEAN = false>
 static int launch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
   using Cfg = HaloCfg<BLOCK_N, PLANES, PITCH, SPLIT, LEAN>;
@@ -325,28 +328,28 @@ static int launch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
   auto kern = conv3x3_halo_kernel<BLOCK_N, PLANES, PITCH, SPLIT, LEAN>;
   static uint64_t attr_done = 0;   // per instantiation: bit d = device d has the shared-memory opt-in
   OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, Cfg::kSmemBytes, &attr_done));
-  const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-  OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(64 + EpiCfg<BLOCK_N>::kThreads), Cfg::kSmemBytes, stream, mx_hi, mx_lo,
+  OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(halo_grid(p.total_tiles, sms)), dim3(64 + EpiCfg<BLOCK_N>::kThreads), Cfg::kSmemBytes, stream, mx_hi, mx_lo,
                               mw_hi, mw_lo, p));
   return OSVOS_OK;
 }
 
-template <int PITCH>
-static int dispatch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
+// What dispatch_halo launches: the instantiation and the persistent grid.  One pure function of the arguments, the SM
+// count and the switches, so that osvos_conv3x3_plan reports exactly what osvos_conv3x3 runs.
+struct HaloChoice {
+  int block_n, planes;
+  bool split, lean;
+};
+static HaloChoice choose_halo(const osvos_conv3x3_args* a, int sms, const HaloSwitches& sw) {
   const bool fast = (a->flags & OSVOS_FLAG_FAST) != 0;
-  const HaloSwitches sw = halo_switches();
-  if (a->cout == 16) return fast ? launch_halo<16, 1, PITCH>(a, stream) : launch_halo<16, 2, PITCH>(a, stream);
+  if (a->cout == 16) return fast ? HaloChoice{16, 1, false, false} : HaloChoice{16, 2, true, false};
   // the lean epilogue serves launches that use nothing but bias / ReLU / split-bf16 act output / fused pool (exact mode)
   const bool lean = sw.lean && !fast && !(a->flags & OSVOS_FLAG_RELU_MASK) && a->colsum == nullptr && a->y_f32 == nullptr &&
                     a->pq == nullptr && (a->y_hi != nullptr || a->pool_hi != nullptr) &&
                     (a->y_hi == nullptr || a->y_lo != nullptr) && (a->pool_hi == nullptr || a->pool_lo != nullptr) &&
                     a->k_valid == 0;
-  if (a->cout == 64) {
-    if (lean) return launch_halo<64, 2, PITCH, true, true>(a, stream);
-    return fast ? launch_halo<64, 1, PITCH>(a, stream) : launch_halo<64, 2, PITCH>(a, stream);
-  }
+  const HaloChoice n64 = lean ? HaloChoice{64, 2, true, true} : fast ? HaloChoice{64, 1, false, false} : HaloChoice{64, 2, true, false};
+  if (a->cout == 64) return n64;
   const int m_tiles = ((a->w + kTileW - 1) / kTileW) * ((a->h + kTileH - 1) / kTileH) * a->n;
-  const int sms = device_sm_count();
   const long tiles128 = static_cast<long>(m_tiles) * (a->cout / 128);
   const long waves128 = (tiles128 + sms - 1) / sms;
   const long waves256 = (static_cast<long>(m_tiles) * (a->cout / 256) + sms - 1) / sms;
@@ -356,22 +359,40 @@ static int dispatch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
   // applied to every badly quantised layer, -1 % / +-0 / +2 % (240p / 480p / 720p) when restricted to layers with at
   // least one whole tile per CTA.  The layers it would help are power-limited: the idle SMs of a ragged last wave are
   // what lets the busy ones clock higher.  Removed again; profiles/r02c_ab_matrix.txt, r02d_ab_matrix_*.txt.)
-  if (waves128 == 1 && tiles128 * 5 <= static_cast<long>(sms) * 3) {
-    if (lean) return launch_halo<64, 2, PITCH, true, true>(a, stream);
-    return fast ? launch_halo<64, 1, PITCH>(a, stream) : launch_halo<64, 2, PITCH>(a, stream);
-  }
+  if (waves128 == 1 && tiles128 * 5 <= static_cast<long>(sms) * 3) return n64;
   // N = 256 tiles (one tcgen05.mma of 128 cycles per pass) whenever that does not cost a wave; measured cycles per
-  // (tap, 64-channel) step: N = 128 ~ 1000 (2 + 1 instructions), N = 256 ~ 2200 exact
+  // (tap, 64-channel) step: N = 128 ~ 1000 (2 + 1 instructions), N = 256 ~ 2200 exact.  (Exact mode never prefers
+  // them: waves128 <= 2 * waves256 whenever cout % 256 == 0.)
   const bool prefer256 = fast ? waves256 * 1100 < waves128 * 700 : waves256 * 2200 < waves128 * 1000;
-  if (a->cout % 256 == 0 && prefer256 && sw.n256)
-    return fast ? launch_halo<256, 1, PITCH>(a, stream) : launch_halo<256, 2, PITCH>(a, stream);
-  if (fast) return launch_halo<128, 1, PITCH>(a, stream);
+  if (a->cout % 256 == 0 && prefer256 && sw.n256) return fast ? HaloChoice{256, 1, false, false} : HaloChoice{256, 2, false, false};
+  if (fast) return HaloChoice{128, 1, false, false};
   // Exact mode, N = 128: the N-concatenated split accumulator (2 MMAs per K step, 256 accumulator columns, the
   // epilogue sums two halves) and the plain three-pass form (3 MMAs, 128 columns) cost the SAME tensor time
   // (scripts/microbench/operand_reuse_bench.cu) and measured the same; OSVOS_SPLITACC128=0 selects the three-pass form.
-  if (!sw.splitacc128) return launch_halo<128, 2, PITCH, false>(a, stream);
-  if (lean) return launch_halo<128, 2, PITCH, true, true>(a, stream);
-  return launch_halo<128, 2, PITCH>(a, stream);
+  if (!sw.splitacc128) return HaloChoice{128, 2, false, false};
+  return HaloChoice{128, 2, true, lean};
+}
+
+template <int PITCH>
+static int dispatch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
+  const HaloChoice c = choose_halo(a, device_sm_count(), halo_switches());
+#define OSVOS_HALO_CASE(BN, PL, SP, LE) \
+  if (c.block_n == BN && c.planes == PL && c.split == SP && c.lean == LE) return launch_halo<BN, PL, PITCH, SP, LE>(a, stream)
+  OSVOS_HALO_CASE(16, 1, false, false);
+  OSVOS_HALO_CASE(16, 2, true, false);
+  OSVOS_HALO_CASE(64, 1, false, false);
+  OSVOS_HALO_CASE(64, 2, true, false);
+  OSVOS_HALO_CASE(64, 2, true, true);
+  OSVOS_HALO_CASE(128, 1, false, false);
+  OSVOS_HALO_CASE(128, 2, false, false);
+  OSVOS_HALO_CASE(128, 2, true, false);
+  OSVOS_HALO_CASE(128, 2, true, true);
+  OSVOS_HALO_CASE(256, 1, false, false);
+  OSVOS_HALO_CASE(256, 2, false, false);
+#undef OSVOS_HALO_CASE
+  set_last_error("conv3x3: no halo instantiation for N = %d, %d plane(s), split %d, lean %d", c.block_n, c.planes,
+                 (int)c.split, (int)c.lean);
+  return OSVOS_ERR_UNSUPPORTED;
 }
 
 int conv3x3_halo_dispatch(const osvos_conv3x3_args* a, cudaStream_t stream) {
@@ -432,20 +453,47 @@ extern "C" int osvos_side_folded_multi(const osvos_conv3x3_args* args, int count
   return side_conv_multi_dispatch(order, count, static_cast<cudaStream_t>(stream_));
 }
 
-extern "C" int osvos_conv3x3(const osvos_conv3x3_args* a, osvos_stream_t stream_) {
-  int rc = check_conv_args(a);
-  if (rc) return rc;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  // side_prep shape (16 outputs, fp32 features / projections only): nine-taps-along-N kernel (side_conv.cu);
-  // OSVOS_SIDE_IMPL=generic sends it through the halo kernel's N = 16 instantiation instead (cross-check)
-  if (a->cout == 2) return side_conv_dispatch(a, stream);
+// side_prep shape (16 outputs, fp32 features / projections only): nine-taps-along-N kernel (side_conv.cu);
+// OSVOS_SIDE_IMPL=generic sends it through the halo kernel's N = 16 instantiation instead (cross-check)
+static bool routes_to_side_conv(const osvos_conv3x3_args* a) {
+  if (a->cout == 2) return true;
   if (a->cout == 16 && a->y_hi == nullptr && !(a->flags & OSVOS_FLAG_RELU_MASK) && a->colsum == nullptr) {
     static int generic = -1;
     if (generic < 0) {
       const char* side = getenv("OSVOS_SIDE_IMPL");
       generic = (side != nullptr && strcmp(side, "generic") == 0) ? 1 : 0;
     }
-    if (!generic) return side_conv_dispatch(a, stream);
+    return !generic;
   }
+  return false;
+}
+
+extern "C" int osvos_conv3x3(const osvos_conv3x3_args* a, osvos_stream_t stream_) {
+  int rc = check_conv_args(a);
+  if (rc) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (routes_to_side_conv(a)) return side_conv_dispatch(a, stream);
   return conv3x3_halo_dispatch(a, stream);
+}
+
+extern "C" int osvos_conv3x3_plan(const osvos_conv3x3_args* a, osvos_launch_plan* plan) {
+  int rc = check_conv_args(a);
+  if (rc) return rc;
+  OSVOS_CHECK_ARG(plan != nullptr);
+  if (routes_to_side_conv(a)) {
+    set_last_error("osvos_conv3x3_plan: these arguments go to the side-branch kernel (side_conv.cu), not the halo kernel");
+    return OSVOS_ERR_UNSUPPORTED;
+  }
+  const int sms = device_sm_count();
+  const HaloChoice c = choose_halo(a, sms, halo_switches());
+  memset(plan, 0, sizeof(*plan));
+  plan->block_n = c.block_n;
+  plan->planes = c.planes;
+  plan->split_acc = c.split ? 1 : 0;
+  plan->lean = c.lean ? 1 : 0;
+  ConvParams p;
+  fill_conv_params(p, a, c.block_n);
+  plan->items = p.total_tiles;
+  plan->grid = halo_grid(p.total_tiles, sms);
+  return OSVOS_OK;
 }

@@ -22,6 +22,7 @@
 // Replaces autograd's weight gradient of nn.Conv2d(k=3, p=1)
 // (reference networks/vgg_osvos.py:41,142; backward triggered at train_online.py:141).
 #include <stdlib.h>
+#include <string.h>
 
 #include "common.cuh"
 #include "ptx.cuh"
@@ -380,19 +381,31 @@ wgrad_finish_multi_kernel(const __grid_constant__ FinishTable t) {
   }
 }
 
-template <int BLOCK_N, int PLANES>
-static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
-  using Cfg = WgCfg<BLOCK_N, PLANES>;
-  // operand roles
-  const void* p_hi = a->dz_hi;
-  const void* p_lo = a->dz_lo;
-  const void* q_hi = a->x_hi;
-  const void* q_lo = a->x_lo;
+// Environment switches of launch_wgrad (A/B; read once).
+struct WgradSwitches {
+  bool rows;          // OSVOS_WGRAD_ROWS     (default 1): tap rows for Cin = Cout = 64; 0: tap pairs instead
+  bool legacy_split;  // OSVOS_WGRAD_SPLITS=legacy: the first split rule
+};
+static WgradSwitches wgrad_switches() {
+  static int rows_on = -1, split_rule = -1;
+  if (rows_on < 0) {
+    const char* e = getenv("OSVOS_WGRAD_ROWS");
+    rows_on = (e == nullptr || atoi(e) != 0) ? 1 : 0;
+  }
+  if (split_rule < 0) {
+    const char* e = getenv("OSVOS_WGRAD_SPLITS");
+    split_rule = (e != nullptr && strcmp(e, "legacy") == 0) ? 1 : 0;
+  }
+  return WgradSwitches{rows_on == 1, split_rule == 1};
+}
+
+// The work decomposition of one launch: every WgradParams field that is not a pointer or an image dimension, and the
+// persistent grid.  One pure function of the arguments, the SM count and the switches, so that
+// osvos_conv3x3_wgrad_plan reports exactly what osvos_conv3x3_wgrad runs.  Returns OSVOS_ERR_UNSUPPORTED for a dz
+// channel count the kernel cannot tile.
+static int plan_wgrad(const osvos_wgrad_args* a, int block_n, int sms, const WgradSwitches& sw, WgradParams& p, int& grid) {
   const int cp = a->dz_channels;   // channels of the P tensor
   const int cq = a->cin;           // channels of the Q tensor
-
-  WgradParams p;
-  p.ws = a->workspace;
   p.n_img = a->n;
   p.h = a->h;
   p.w = a->w;
@@ -409,33 +422,22 @@ static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
   // instead of the two of four of tap pairs under a half-empty M (a tcgen05.mma costs max(M, 128) rows either way).
   // Exact at the borders: the terms dz[u] x[u + (., -1)] the shifted M atom cannot reach (u.x = 0) multiply the zero
   // padding of x, and everything out of the image is zero-filled by TMA on both operands.
-  static int rows_on = -1;   // OSVOS_WGRAD_ROWS=0: tap pairs instead (A/B; read once)
-  if (rows_on < 0) {
-    const char* e = getenv("OSVOS_WGRAD_ROWS");
-    rows_on = (e == nullptr || atoi(e) != 0) ? 1 : 0;
-  }
-  p.tap_rows = (rows_on && cq == 64 && cp == 64 && BLOCK_N == 128) ? 1 : 0;
-  p.tap_pairs = (cq == 64 && BLOCK_N == 128 && !p.tap_rows) ? 1 : 0;
+  p.tap_rows = (sw.rows && cq == 64 && cp == 64 && block_n == 128) ? 1 : 0;
+  p.tap_pairs = (cq == 64 && block_n == 128 && !p.tap_rows) ? 1 : 0;
   p.tap_items = p.tap_rows ? 3 : p.tap_pairs ? 5 : 9;
-  p.n_blocks = (p.tap_pairs || p.tap_rows) ? 1 : cq / BLOCK_N;
+  p.n_blocks = (p.tap_pairs || p.tap_rows) ? 1 : cq / block_n;
   p.patches_x = (a->w + kWgPatchW - 1) / kWgPatchW;
   p.patches_y = (a->h + kWgPatchH - 1) / kWgPatchH;
   p.patches_total = p.patches_x * p.patches_y * a->n;
   const int tiles = p.m_blocks * p.n_blocks * p.tap_items;
-  const int sms = device_sm_count();
   // Pixel-range splits: items are dealt round-robin to the persistent CTAs, so the kernel lasts as long as the CTA with
   // the most items - ROUNDS x K blocks per item.  Pick the split count that minimises that (plus ~2 K-block times per
   // item for the accumulator flush that is not hidden behind the next item's MMAs).  The first rule, ceil(2 SMs /
   // tiles), landed just ABOVE two full rounds for most layers (297 items on 148 CTAs: a third round for one item,
   // 67 % of the tensor time) - profiles/r02l_*.
   const int max_splits = (p.patches_total + 3) / 4;
-  static int split_rule = -1;   // OSVOS_WGRAD_SPLITS=legacy: the first rule (A/B; read once)
-  if (split_rule < 0) {
-    const char* e = getenv("OSVOS_WGRAD_SPLITS");
-    split_rule = (e != nullptr && strcmp(e, "legacy") == 0) ? 1 : 0;
-  }
   int splits = 1;
-  if (split_rule == 1) {
+  if (sw.legacy_split) {
     splits = (2 * sms + tiles - 1) / tiles;
   } else {
     long best = -1;
@@ -456,6 +458,26 @@ static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
   p.patches_per_split = (p.patches_total + splits - 1) / splits;
   p.splits = (p.patches_total + p.patches_per_split - 1) / p.patches_per_split;
   p.total_items = tiles * p.splits;
+  grid = p.total_items < sms ? p.total_items : sms;
+  return OSVOS_OK;
+}
+
+template <int BLOCK_N, int PLANES>
+static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
+  using Cfg = WgCfg<BLOCK_N, PLANES>;
+  // operand roles
+  const void* p_hi = a->dz_hi;
+  const void* p_lo = a->dz_lo;
+  const void* q_hi = a->x_hi;
+  const void* q_lo = a->x_lo;
+  const int cp = a->dz_channels;   // channels of the P tensor
+  const int cq = a->cin;           // channels of the Q tensor
+
+  WgradParams p;
+  int grid = 0;
+  const int rc_plan = plan_wgrad(a, BLOCK_N, device_sm_count(), wgrad_switches(), p, grid);
+  if (rc_plan) return rc_plan;
+  p.ws = a->workspace;
 
   CUtensorMap mp_hi, mp_lo, mq_hi, mq_lo;
   auto enc = [&](CUtensorMap* m, const void* base, int c) {
@@ -477,7 +499,6 @@ static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
   auto kern = wgrad_tc_kernel<BLOCK_N, PLANES>;
   static uint64_t attr_done = 0;   // per instantiation: bit d = device d has the shared-memory opt-in
   OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, Cfg::kSmemBytes, &attr_done));
-  const int grid = p.total_items < sms ? p.total_items : sms;
   if (deferred) {   // (otherwise the memset above is this kernel's stream predecessor: plain launch)
     OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kWgThreads), Cfg::kSmemBytes, stream, mp_hi, mp_lo, mq_hi, mq_lo, p));
     return OSVOS_OK;
@@ -528,14 +549,45 @@ extern "C" int osvos_wgrad_finish(const osvos_wgrad_finish_item* items, int coun
   return OSVOS_OK;
 }
 
-extern "C" int osvos_conv3x3_wgrad(const osvos_wgrad_args* a, osvos_stream_t stream_) {
+static int check_wgrad_args(const osvos_wgrad_args* a) {
   OSVOS_CHECK_ARG(a != nullptr && a->x_hi != nullptr && a->dz_hi != nullptr && a->workspace != nullptr);
   OSVOS_CHECK_ARG(a->dw != nullptr || (a->flags & OSVOS_FLAG_DEFER_FINISH));
   OSVOS_CHECK_ARG(a->n > 0 && a->h > 0 && a->w > 0 && a->cin % 64 == 0 && a->dz_channels % 64 == 0);
   OSVOS_CHECK_ARG(a->cout == a->dz_channels);
   OSVOS_CHECK_ARG((a->flags & OSVOS_FLAG_FAST) || (a->x_lo != nullptr && a->dz_lo != nullptr));
   OSVOS_CHECK_ARG(a->cin % 128 == 0 || a->cin == 64);     // Cin = 64: tap-pair / tap-row modes of the 128-wide kernel
+  return OSVOS_OK;
+}
+
+extern "C" int osvos_conv3x3_wgrad(const osvos_wgrad_args* a, osvos_stream_t stream_) {
+  int rc = check_wgrad_args(a);
+  if (rc) return rc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   const bool fast = (a->flags & OSVOS_FLAG_FAST) != 0;
   return fast ? launch_wgrad<128, 1>(a, stream) : launch_wgrad<128, 2>(a, stream);
+}
+
+extern "C" int osvos_conv3x3_wgrad_plan(const osvos_wgrad_args* a, osvos_launch_plan* plan) {
+  int rc = check_wgrad_args(a);
+  if (rc) return rc;
+  OSVOS_CHECK_ARG(plan != nullptr);
+  const bool fast = (a->flags & OSVOS_FLAG_FAST) != 0;
+  constexpr int kBlockN = 128;   // the only instantiation width (osvos_conv3x3_wgrad above)
+  WgradParams p;
+  int grid = 0;
+  rc = plan_wgrad(a, kBlockN, device_sm_count(), wgrad_switches(), p, grid);
+  if (rc) {
+    set_last_error("osvos_conv3x3_wgrad_plan: dz_channels = %d cannot be tiled", a->dz_channels);
+    return rc;
+  }
+  memset(plan, 0, sizeof(*plan));
+  plan->block_n = kBlockN;
+  plan->planes = fast ? 1 : 2;
+  plan->split_acc = fast ? WgCfg<kBlockN, 1>::kSplitAcc : WgCfg<kBlockN, 2>::kSplitAcc;
+  plan->lean = 0;
+  plan->items = p.total_items;
+  plan->grid = grid;
+  plan->tap_mode = p.tap_rows ? OSVOS_TAP_ROWS : p.tap_pairs ? OSVOS_TAP_PAIRS : OSVOS_TAP_NINE;
+  plan->pixel_splits = p.splits;
+  return OSVOS_OK;
 }

@@ -191,12 +191,8 @@ def side_folded_multi(xs, folded, fast=False):
     return pqs
 
 
-def conv3x3(x, w_packed, bias, cout, relu=False, fast=False, out_act=True, out_f32=False, mask=None,
-            proj_w=None, proj_b=None, simt=False, pool=False, colsum=None, k_valid=0):
-    """3x3 / pad 1 conv of an Act through the tcgen05 kernel.  Returns (Act|None, f32|None, pq|None), or
-    (Act, pooled Act) when pool=True (fused MaxPool2d(2,2,ceil_mode)).  `colsum` ([cout] fp32, pre-zeroed)
-    receives the per-channel sum of the output (fused bias gradient)."""
-    lib = nat.load()
+def _conv3x3_call(x, w_packed, bias, cout, relu, fast, out_act, out_f32, mask, proj_w, proj_b, pool, colsum, k_valid):
+    """Outputs and the osvos_conv3x3_args block of one conv3x3 call -> (args, y, yf, pq, yp)."""
     n, h, w, cin = x.shape
     dev = x.hi.device
     y = Act.empty(n, h, w, cout, dev, fast) if out_act else None
@@ -218,12 +214,39 @@ def conv3x3(x, w_packed, bias, cout, relu=False, fast=False, out_act=True, out_f
     a.n, a.h, a.w, a.cin, a.cout = n, h, w, cin, cout
     a.flags = (nat.FLAG_RELU if relu else 0) | (nat.FLAG_FAST if fast else 0) | \
               (nat.FLAG_RELU_MASK if mask is not None else 0)
+    return a, y, yf, pq, yp
+
+
+def conv3x3(x, w_packed, bias, cout, relu=False, fast=False, out_act=True, out_f32=False, mask=None,
+            proj_w=None, proj_b=None, simt=False, pool=False, colsum=None, k_valid=0):
+    """3x3 / pad 1 conv of an Act through the tcgen05 kernel.  Returns (Act|None, f32|None, pq|None), or
+    (Act, pooled Act) when pool=True (fused MaxPool2d(2,2,ceil_mode)).  `colsum` ([cout] fp32, pre-zeroed)
+    receives the per-channel sum of the output (fused bias gradient)."""
+    lib = nat.load()
+    a, y, yf, pq, yp = _conv3x3_call(x, w_packed, bias, cout, relu, fast, out_act, out_f32, mask, proj_w, proj_b, pool,
+                                     colsum, k_valid)
     fn = lib.osvos_conv3x3_simt if simt else lib.osvos_conv3x3
     _count()
     nat.check(fn(byref(a), _stream()), "osvos_conv3x3")
     if pool:
         return y, yp
     return y, yf, pq
+
+
+def _plan_dict(plan):
+    return {name: int(getattr(plan, name)) for name, _ in nat.LaunchPlan._fields_}
+
+
+def conv3x3_plan(x, w_packed, bias, cout, relu=False, fast=False, out_act=True, out_f32=False, mask=None,
+                 proj_w=None, proj_b=None, pool=False, colsum=None, k_valid=0):
+    """The launch plan (osvos_conv3x3_plan) of the conv3x3 call with the same arguments, as a dict: block_n, planes,
+    split_acc, lean, items, grid (tap_mode and pixel_splits are 0).  Nothing is launched."""
+    lib = nat.load()
+    a, *_ = _conv3x3_call(x, w_packed, bias, cout, relu, fast, out_act, out_f32, mask, proj_w, proj_b, pool, colsum,
+                          k_valid)
+    plan = nat.LaunchPlan()
+    nat.check(lib.osvos_conv3x3_plan(byref(a), byref(plan)), "osvos_conv3x3_plan")
+    return _plan_dict(plan)
 
 
 def maxpool2x2(x):
@@ -313,30 +336,45 @@ def wgrad_workspace_floats(dz_channels, cin):
     return nat.load().osvos_wgrad_workspace_bytes(dz_channels, cin) // 4
 
 
+def _wgrad_args(x, dz, cout, fast):
+    n, h, w, cin = x.shape
+    a = nat.WgradArgs()
+    a.x_hi, a.x_lo, a.dz_hi, a.dz_lo = x.hi.data_ptr(), nat.ptr(x.lo), dz.hi.data_ptr(), nat.ptr(dz.lo)
+    a.n, a.h, a.w, a.cin, a.cout, a.dz_channels = n, h, w, cin, cout, dz.shape[3]
+    a.flags = nat.FLAG_FAST if fast else 0
+    return a
+
+
 def conv3x3_wgrad(x, dz, cout, fast=False, deferred_ws=None):
     """dW [cout, cin, 3, 3] of a 3x3 conv from its input act `x` and output-gradient act `dz`.
     With `deferred_ws` (a ZEROED fp32 workspace of wgrad_workspace_floats(dz.channels, cin)) only the tensor-core
     accumulation is enqueued and a finish item for ops.wgrad_finish is returned instead of dW."""
     lib = nat.load()
-    n, h, w, cin = x.shape
-    dzc = dz.shape[3]
-    dev = x.hi.device
-    a = nat.WgradArgs()
-    a.x_hi, a.x_lo, a.dz_hi, a.dz_lo = x.hi.data_ptr(), nat.ptr(x.lo), dz.hi.data_ptr(), nat.ptr(dz.lo)
-    a.n, a.h, a.w, a.cin, a.cout, a.dz_channels = n, h, w, cin, cout, dzc
-    a.flags = nat.FLAG_FAST if fast else 0
+    cin, dzc = x.shape[3], dz.shape[3]
+    a = _wgrad_args(x, dz, cout, fast)
     if deferred_ws is not None:
         a.dw, a.workspace = None, deferred_ws.data_ptr()
         a.flags |= nat.FLAG_DEFER_FINISH
         _count(1)
         nat.check(lib.osvos_conv3x3_wgrad(byref(a), _stream()), "osvos_conv3x3_wgrad")
         return {"ws": deferred_ws, "cout": cout, "cin": cin, "dz_channels": dzc}
-    dw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=dev)
-    ws = torch.empty(lib.osvos_wgrad_workspace_bytes(dzc, cin) // 4, dtype=torch.float32, device=dev)
+    dw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=x.hi.device)
+    ws = torch.empty(lib.osvos_wgrad_workspace_bytes(dzc, cin) // 4, dtype=torch.float32, device=x.hi.device)
     a.dw, a.workspace = dw.data_ptr(), ws.data_ptr()
     _count(3)
     nat.check(lib.osvos_conv3x3_wgrad(byref(a), _stream()), "osvos_conv3x3_wgrad")
     return dw
+
+
+def conv3x3_wgrad_plan(x, dz, cout, fast=False):
+    """The launch plan (osvos_conv3x3_wgrad_plan) of conv3x3_wgrad(x, dz, cout, fast) as a dict: block_n, planes,
+    split_acc, lean, items, grid, tap_mode (nat.TAP_ROWS / TAP_PAIRS / TAP_NINE), pixel_splits.  Nothing is launched."""
+    lib = nat.load()
+    a = _wgrad_args(x, dz, cout, fast)
+    a.dw = a.workspace = x.hi.data_ptr()     # required non-NULL by the argument check; never written by the query
+    plan = nat.LaunchPlan()
+    nat.check(lib.osvos_conv3x3_wgrad_plan(byref(a), byref(plan)), "osvos_conv3x3_wgrad_plan")
+    return _plan_dict(plan)
 
 
 def wgrad_finish(items):
