@@ -464,9 +464,8 @@ static int launch_unpool(const void* dpool_hi, const void* dpool_lo, const void*
   // the folded weights go to shared memory when every block has tiles enough to amortise the copy
   const int wf_in_smem = (SIDE && tiles >= static_cast<size_t>(grid) * 4) ? 1 : 0;
   const size_t smem = static_cast<size_t>(c) * sizeof(float) * (wf_in_smem ? 19 : 1);
-  auto kern = unpool_add_mask_kernel<POOL, SIDE>;
-  static uint64_t attr_done = 0;
-  if (smem > 48 * 1024) OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, 19 * 2048 * sizeof(float), &attr_done));
+  constexpr auto kern = unpool_add_mask_kernel<POOL, SIDE>;
+  if (smem > 48 * 1024) OSVOS_CHECK_CUDA(ensure_dynamic_smem<kern>(19 * 2048 * sizeof(float)));
   OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(256), smem, stream,
                               static_cast<const __nv_bfloat16*>(dpool_hi), static_cast<const __nv_bfloat16*>(dpool_lo),
                               static_cast<const __nv_bfloat16*>(x_hi), static_cast<const __nv_bfloat16*>(x_lo), dside, dpq,

@@ -1,12 +1,13 @@
 // 3x3 convolution as a tcgen05 implicit GEMM with HALO REUSE (sm_100a).
 //
-// Same GEMM view, tile geometry, precision scheme, warp roles and epilogue as conv3x3_tc.cu, but the
-// activation operand is loaded ONCE per (tile, 64-channel chunk) as the 18-row x 10-px halo patch and the
-// nine taps are nine UMMA smem descriptors into it: tap (r, s) starts at smem row (r * PITCH + s); the 16
-// tile rows are the sixteen 8-row swizzle groups at stride SBO = PITCH * 128 B.  That divides the
-// activation traffic through L2 -> smem by ~6 relative to one shifted box per tap, which is what bounded
-// the per-tap kernel (DESIGN.md section 4).  The weight slabs stream through their own, deeper ring
-// (one stage per tap), and the next chunk's halo is prefetched while the current one is being consumed.
+// GEMM view: M = 128 output pixels (8 px x 16 rows), N = BLOCK_N output channels, K = 9 taps x Cin; split-bf16
+// operands; warp 0 is the TMA producer, warp 1 the MMA issuer, the others run the epilogue (conv_common.cuh).
+// The activation operand is loaded ONCE per (tile, 64-channel chunk) as the 18-row x 10-px halo patch and the nine taps
+// are nine UMMA smem descriptors into it: tap (r, s) starts at smem row (r * PITCH + s); the 16 tile rows are the sixteen
+// 8-row swizzle groups at stride SBO = PITCH * 128 B.  That divides the activation traffic through L2 -> smem by ~6
+// relative to one shifted box per tap, which is what bounded the earlier per-tap kernel (DESIGN.md section 4).  The
+// weight slabs stream through their own, deeper ring (one stage per tap), and the next chunk's halo is prefetched while
+// the current one is being consumed.
 //
 // PITCH is the smem row pitch in pixels: 10 packs the patch rows (1280 B) and relies on the UMMA swizzle being a
 // function of the absolute shared-memory address, validated on hardware together with the padded 16-pixel pitch and the
@@ -14,7 +15,6 @@
 //
 // Producer and issuer loops: one elected thread each, taps unrolled, descriptors by addition - see the comments at
 // the two loops and DESIGN.md section 4 for the measurements behind that.
-#include <stdlib.h>
 #include <string.h>
 
 #include <type_traits>
@@ -278,58 +278,28 @@ conv3x3_halo_kernel(const __grid_constant__ CUtensorMap map_x_hi, const __grid_c
   }
 }
 
-// Environment switches of the dispatcher (A/B and diagnosis; defaults are the measured winners).  Read ONCE per process;
-// OSVOS_ENV_RELOAD=1 makes every dispatch re-read them (scripts/ab_env.py flips switches inside one process).
+// The dispatcher's switches: OSVOS_HALO_LEAN, OSVOS_CONV_N256, OSVOS_SPLITACC128 (runtime.cu).
 struct HaloSwitches {
-  bool lean;        // OSVOS_HALO_LEAN      (default 1): lean epilogue for plain forward launches
-  bool n256;        // OSVOS_CONV_N256      (default 1): 256-wide tiles where they pay
-  bool splitacc128; // OSVOS_SPLITACC128    (default 1): N-concatenated accumulator for 128-wide exact tiles
+  bool lean, n256, splitacc128;
 };
-static bool env_flag(const char* name, bool dflt) {
-  const char* e = getenv(name);
-  return e == nullptr ? dflt : atoi(e) != 0;
-}
 static HaloSwitches halo_switches() {
-  static HaloSwitches sw;
-  static int state = 0;          // 0: unread, 1: cached, 2: re-read on every call
-  if (state != 1) {
-    sw.lean = env_flag("OSVOS_HALO_LEAN", true);
-    sw.n256 = env_flag("OSVOS_CONV_N256", true);
-    sw.splitacc128 = env_flag("OSVOS_SPLITACC128", true);
-    state = env_flag("OSVOS_ENV_RELOAD", false) ? 2 : 1;
-  }
-  return sw;
+  return HaloSwitches{env_int("OSVOS_HALO_LEAN", 1) != 0, env_int("OSVOS_CONV_N256", 1) != 0,
+                      env_int("OSVOS_SPLITACC128", 1) != 0};
 }
-
-// persistent CTAs: one per tile up to one per SM; CTA b takes tiles b, b + grid, b + 2 grid, ...
-static int halo_grid(int tiles, int sms) { return tiles < sms ? tiles : sms; }
 
 template <int BLOCK_N, int PLANES, int PITCH, bool SPLIT = (PLANES == 2 && BLOCK_N <= 128), bool LEAN = false>
 static int launch_halo(const osvos_conv3x3_args* a, cudaStream_t stream) {
   using Cfg = HaloCfg<BLOCK_N, PLANES, PITCH, SPLIT, LEAN>;
   ConvParams p;
   fill_conv_params(p, a, BLOCK_N);
-  const int sms = device_sm_count();
   CUtensorMap mx_hi, mx_lo, mw_hi, mw_lo;
-  {
-    const uint64_t dims[4] = {(uint64_t)a->cin, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-    const uint64_t strides[3] = {(uint64_t)a->cin * 2, (uint64_t)a->w * a->cin * 2,
-                                 (uint64_t)a->h * a->w * a->cin * 2};
-    const uint32_t box[4] = {kBlockK, PITCH, kHaloRows, 1};
-    int rc = encode_tensor_map(&mx_hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, a->x_hi, dims, strides, box,
-                               CU_TENSOR_MAP_SWIZZLE_128B);
-    if (rc) return rc;
-    rc = encode_tensor_map(&mx_lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, PLANES == 2 ? a->x_lo : a->x_hi, dims,
-                           strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
-    if (rc) return rc;
-  }
-  int rc = encode_weight_maps(&mw_hi, &mw_lo, a, BLOCK_N);
+  int rc = encode_act_maps(&mx_hi, &mx_lo, a->x_hi, PLANES == 2 ? a->x_lo : nullptr, a->n, a->h, a->w, a->cin, PITCH,
+                           kHaloRows);
   if (rc) return rc;
-  auto kern = conv3x3_halo_kernel<BLOCK_N, PLANES, PITCH, SPLIT, LEAN>;
-  static uint64_t attr_done = 0;   // per instantiation: bit d = device d has the shared-memory opt-in
-  OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, Cfg::kSmemBytes, &attr_done));
-  OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(halo_grid(p.total_tiles, sms)), dim3(64 + EpiCfg<BLOCK_N>::kThreads), Cfg::kSmemBytes, stream, mx_hi, mx_lo,
-                              mw_hi, mw_lo, p));
+  rc = encode_weight_maps(&mw_hi, &mw_lo, a->w_packed, a->cout, a->cin, BLOCK_N, 1);
+  if (rc) return rc;
+  OSVOS_CHECK_CUDA((launch_persistent<conv3x3_halo_kernel<BLOCK_N, PLANES, PITCH, SPLIT, LEAN>>(
+      p.total_tiles, 64 + EpiCfg<BLOCK_N>::kThreads, Cfg::kSmemBytes, stream, mx_hi, mx_lo, mw_hi, mw_lo, p)));
   return OSVOS_OK;
 }
 
@@ -457,15 +427,8 @@ extern "C" int osvos_side_folded_multi(const osvos_conv3x3_args* args, int count
 // OSVOS_SIDE_IMPL=generic sends it through the halo kernel's N = 16 instantiation instead (cross-check)
 static bool routes_to_side_conv(const osvos_conv3x3_args* a) {
   if (a->cout == 2) return true;
-  if (a->cout == 16 && a->y_hi == nullptr && !(a->flags & OSVOS_FLAG_RELU_MASK) && a->colsum == nullptr) {
-    static int generic = -1;
-    if (generic < 0) {
-      const char* side = getenv("OSVOS_SIDE_IMPL");
-      generic = (side != nullptr && strcmp(side, "generic") == 0) ? 1 : 0;
-    }
-    return !generic;
-  }
-  return false;
+  return a->cout == 16 && a->y_hi == nullptr && !(a->flags & OSVOS_FLAG_RELU_MASK) && a->colsum == nullptr &&
+         !env_is("OSVOS_SIDE_IMPL", "generic");
 }
 
 extern "C" int osvos_conv3x3(const osvos_conv3x3_args* a, osvos_stream_t stream_) {
@@ -494,6 +457,6 @@ extern "C" int osvos_conv3x3_plan(const osvos_conv3x3_args* a, osvos_launch_plan
   ConvParams p;
   fill_conv_params(p, a, c.block_n);
   plan->items = p.total_tiles;
-  plan->grid = halo_grid(p.total_tiles, sms);
+  plan->grid = persistent_grid(p.total_tiles, sms);
   return OSVOS_OK;
 }

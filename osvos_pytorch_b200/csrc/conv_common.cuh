@@ -1,9 +1,7 @@
-// Shared pieces of the tcgen05 implicit-GEMM convolution kernels (conv3x3_tc.cu: per-tap TMA loads;
-// conv3x3_halo.cu: halo patch loaded once per channel chunk): tile geometry, parameters, tile decode and
-// the epilogue (TMEM -> registers -> bias / ReLU / mask / split-bf16 / projections -> global).
+// Shared pieces of the tcgen05 implicit-GEMM convolution kernels (conv3x3_halo.cu, conv_stage1_fused.cu,
+// conv_first_tc.cu): tile geometry, parameters, tile decode and the epilogue (TMEM -> registers -> bias / ReLU / mask /
+// split-bf16 / projections -> global).
 #pragma once
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -13,7 +11,6 @@ constexpr int kTileW = 8;     // pixels per patch row  (= one 8-row swizzle atom
 constexpr int kTileH = 16;    // patch rows
 constexpr int kBlockM = 128;  // kTileW * kTileH
 constexpr int kBlockK = 64;   // channels per K block (128 B of bf16)
-constexpr int kConvThreads = 192;
 constexpr int kABytes = kBlockM * kBlockK * 2;  // 16 KiB per plane
 
 struct ConvParams {
@@ -30,8 +27,7 @@ struct ConvParams {
   float* colsum;           // optional fused per-channel sum of the output (bias gradient), atomically accumulated
   int n, h, w, cin, cout;
   int tiles_x, tiles_y, n_blocks, total_tiles, k_chunks;
-  int k_steps;               // tcgen05.mma K steps (of 16 channels) issued per 64-channel chunk: 4, or fewer (k_valid)
-  int m_tiles, total_pairs;  // CTA-pair kernels: m_tiles pixel tiles, total_pairs = ceil(m_tiles / 2) * n_blocks work items
+  int k_steps;  // tcgen05.mma K steps (of 16 channels) issued per 64-channel chunk: 4, or fewer (k_valid)
   int flags;
   // Timing ablations (OSVOS_ABLATE bit mask, diagnosis only - results are garbage): 1 = no weight TMA loads,
   // 2 = no activation TMA loads, 4 = no tcgen05.mma, 8 = no global stores in the epilogue.  0 in production.
@@ -307,7 +303,7 @@ __device__ __forceinline__ void conv_epilogue_loop(const ConvParams& p, uint32_t
 //    latency overlaps the split / store / pool work (21 % of the busy samples were waits on the first use);
 //  * the accumulator stage is handed back to the MMA warp right after the LAST tcgen05.ld of the tile has landed,
 //    before the stores - not at the end of the tile;
-//  * no mask / column-sum / fp32 / split-K / bulk-store code: ~1/3 of the instruction footprint next to the issuer.
+//  * no mask / column-sum / fp32 / bulk-store code: ~1/3 of the instruction footprint next to the issuer.
 struct NoTileHook {
   __device__ __forceinline__ void operator()(int) const {}
 };
@@ -422,18 +418,6 @@ __device__ __forceinline__ void conv_epilogue_lean(const ConvParams& p, uint32_t
   }
 }
 
-// Output act [n,h,w,cout] -> 4-D store maps with box {64, kTileW, kTileH, 1} (SWIZZLE_128B); conv1_1's bulk stores.
-static inline int encode_output_maps(CUtensorMap* hi, CUtensorMap* lo, const osvos_conv3x3_args* a) {
-  const uint64_t dims[4] = {(uint64_t)a->cout, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-  const uint64_t strides[3] = {(uint64_t)a->cout * 2, (uint64_t)a->w * a->cout * 2, (uint64_t)a->h * a->w * a->cout * 2};
-  const uint32_t box[4] = {64, kTileW, kTileH, 1};
-  int rc = encode_tensor_map(hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, a->y_hi, dims, strides, box,
-                             CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  return encode_tensor_map(lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, a->y_lo ? a->y_lo : a->y_hi, dims, strides, box,
-                           CU_TENSOR_MAP_SWIZZLE_128B);
-}
-
 // ---- host helpers shared by the launchers ------------------------------------------------
 static inline void fill_conv_params(ConvParams& p, const osvos_conv3x3_args* a, int block_n) {
   p.bias = a->bias;
@@ -456,33 +440,10 @@ static inline void fill_conv_params(ConvParams& p, const osvos_conv3x3_args* a, 
   p.tiles_y = (a->h + kTileH - 1) / kTileH;
   p.n_blocks = a->cout / block_n;
   p.total_tiles = p.tiles_x * p.tiles_y * a->n * p.n_blocks;
-  p.m_tiles = p.tiles_x * p.tiles_y * a->n;
-  p.total_pairs = ((p.m_tiles + 1) / 2) * p.n_blocks;
   p.k_chunks = a->cin / kBlockK;
   p.k_steps = (a->k_valid > 0 && a->k_valid < kBlockK) ? (a->k_valid + 15) / 16 : kBlockK / 16;
   p.flags = a->flags;
-  {
-    static int ablate = -1;
-    if (ablate < 0) {
-      const char* e = getenv("OSVOS_ABLATE");
-      ablate = e ? atoi(e) : 0;
-    }
-    p.ablate = ablate;
-  }
-}
-
-// Packed weights [plane][tap][cout][cin] -> two 3-D maps with box {64, block_n, 1}.
-static inline int encode_weight_maps(CUtensorMap* hi, CUtensorMap* lo, const osvos_conv3x3_args* a, int block_n) {
-  const size_t plane = static_cast<size_t>(9) * a->cout * a->cin;  // elements
-  const uint64_t dims[3] = {(uint64_t)a->cin, (uint64_t)a->cout, 9};
-  const uint64_t strides[2] = {(uint64_t)a->cin * 2, (uint64_t)a->cout * a->cin * 2};
-  const uint32_t box[3] = {kBlockK, (uint32_t)block_n, 1};
-  const __nv_bfloat16* wp = static_cast<const __nv_bfloat16*>(a->w_packed);
-  int rc = encode_tensor_map(hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp, dims, strides, box,
-                             CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  return encode_tensor_map(lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp + plane, dims, strides, box,
-                           CU_TENSOR_MAP_SWIZZLE_128B);
+  p.ablate = env_int("OSVOS_ABLATE", 0);
 }
 
 int conv_first_tc_launch(const float* x, const float* w_oihw, const float* bias, void* y_hi, void* y_lo, int n, int h,

@@ -216,18 +216,14 @@ int conv_first_tc_launch(const float* x, const float* w_oihw, const float* bias,
   a.flags = flags;
   ConvParams p;
   fill_conv_params(p, &a, 64);
-  CUtensorMap my_hi, my_lo;
-  {
-    int rc = encode_output_maps(&my_hi, &my_lo, &a);
-    if (rc) return rc;
-  }
-  const bool fast = (flags & OSVOS_FLAG_FAST) != 0;
-  auto kern = fast ? conv_first_tc_kernel<1> : conv_first_tc_kernel<2>;
-  static uint64_t attr_done[2] = {0, 0};   // per instantiation: bit d = device d has the shared-memory opt-in
-  OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, kFirstSmem, &attr_done[fast ? 1 : 0]));
-  const int sms = device_sm_count();
-  const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-  OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kFirstTcThreads), kFirstSmem, stream, x, w_oihw, my_hi, my_lo, p));
+  CUtensorMap my_hi, my_lo;   // the act output's bulk-store maps
+  const int rc = encode_act_maps(&my_hi, &my_lo, a.y_hi, a.y_lo, n, h, w, 64, kTileW, kTileH);
+  if (rc) return rc;
+  OSVOS_CHECK_CUDA((flags & OSVOS_FLAG_FAST)
+                       ? launch_persistent<conv_first_tc_kernel<1>>(p.total_tiles, kFirstTcThreads, kFirstSmem, stream, x,
+                                                                    w_oihw, my_hi, my_lo, p)
+                       : launch_persistent<conv_first_tc_kernel<2>>(p.total_tiles, kFirstTcThreads, kFirstSmem, stream, x,
+                                                                    w_oihw, my_hi, my_lo, p));
   return OSVOS_OK;
 }
 

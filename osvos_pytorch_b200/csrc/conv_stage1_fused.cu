@@ -24,8 +24,9 @@
 // thread, taps of the next tile and the next 16 accumulator columns requested ahead: 7.5 k.  v3 - one base pointer and
 // 32-bit offsets for the 27 taps instead of per-tap 64-bit addressing: 6.9 k, the stage-1 warps still the pace of the
 // kernel.  v4 (this) - step 1 moved to the epilogue warps, three tiles ahead, so that the stage-1 warps only convert.
-#include <stdlib.h>
 #include <string.h>
+
+#include <type_traits>
 
 #include "conv_common.cuh"
 
@@ -421,25 +422,17 @@ extern "C" int osvos_stage1_fused(const osvos_stage1_args* a, osvos_stream_t str
   ConvParams p;
   fill_conv_params(p, &c, 64);
   CUtensorMap mw_hi, mw_lo;
-  int rc = encode_weight_maps(&mw_hi, &mw_lo, &c, 64);
+  int rc = encode_weight_maps(&mw_hi, &mw_lo, a->w2_packed, 64, 64, 64, 1);
   if (rc) return rc;
   Stage1Params s1;
   s1.x = a->x;
   s1.w1 = a->w1;
   s1.b1 = a->b1;
-  const int sms = device_sm_count();
-  const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-  const char* e = getenv("OSVOS_S1_SW64");                 // 0: 128-byte operand rows + 3-stage weight ring (A/B runs)
-  if (e != nullptr && atoi(e) == 0) {
-    auto kern = conv_stage1_fused_kernel<false>;
-    static uint64_t attr_done = 0;
-    OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, S1Cfg<false>::kSmem, &attr_done));
-    OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kS1Threads), S1Cfg<false>::kSmem, stream, mw_hi, mw_lo, s1, p));
-  } else {
-    auto kern = conv_stage1_fused_kernel<true>;
-    static uint64_t attr_done = 0;
-    OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, S1Cfg<true>::kSmem, &attr_done));
-    OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kS1Threads), S1Cfg<true>::kSmem, stream, mw_hi, mw_lo, s1, p));
-  }
+  auto launch = [&](auto sw64) {
+    constexpr bool SW64 = decltype(sw64)::value;
+    return launch_persistent<conv_stage1_fused_kernel<SW64>>(p.total_tiles, kS1Threads, S1Cfg<SW64>::kSmem, stream, mw_hi,
+                                                             mw_lo, s1, p);
+  };
+  OSVOS_CHECK_CUDA(env_int("OSVOS_S1_SW64", 1) != 0 ? launch(std::true_type{}) : launch(std::false_type{}));
   return OSVOS_OK;
 }

@@ -2,9 +2,6 @@
 // weight packing, NCHW<->act conversion, conv1_1 (Cin = 3), 2x2 ceil-mode max
 // pooling, a CUDA-core reference conv (debug cross-check) and the standalone
 // side-feature projection.
-#include <stdlib.h>
-#include <string.h>
-
 #include "common.cuh"
 
 namespace osvos {
@@ -441,11 +438,9 @@ extern "C" int osvos_conv_first_fwd(const float* x, const float* w_oihw, const f
                                     int n, int h, int w, int flags, osvos_stream_t stream) {
   OSVOS_CHECK_ARG(x != nullptr && w_oihw != nullptr && y_hi != nullptr && n > 0 && h > 0 && w > 0);
   OSVOS_CHECK_ARG(h <= 65535 && n <= 65535);
-  {  // default: tensor-core kernel (conv_first_tc.cu); OSVOS_FIRST_IMPL=simt keeps the CUDA-core one as a cross-check
-    const char* impl = getenv("OSVOS_FIRST_IMPL");
-    if (impl == nullptr || strcmp(impl, "simt") != 0)
-      return conv_first_tc_launch(x, w_oihw, bias, y_hi, y_lo, n, h, w, flags, static_cast<cudaStream_t>(stream));
-  }
+  // the tensor-core kernel (conv_first_tc.cu), unless OSVOS_FIRST_IMPL=simt selects the CUDA-core one as a cross-check
+  if (!env_is("OSVOS_FIRST_IMPL", "simt"))
+    return conv_first_tc_launch(x, w_oihw, bias, y_hi, y_lo, n, h, w, flags, static_cast<cudaStream_t>(stream));
   dim3 grid((w + kFirstThreads - 1) / kFirstThreads, h, n);
   conv_first_kernel<<<grid, kFirstThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       x, w_oihw, bias, static_cast<__nv_bfloat16*>(y_hi),

@@ -18,7 +18,6 @@ namespace osvos {
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
-__device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
 
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred = 0;
@@ -83,19 +82,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// gpu-scope acquire load / release reduction on a global counter (split-K handshake between CTAs)
-__device__ __forceinline__ uint32_t ld_acquire_gpu_u32(const unsigned int* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void red_release_gpu_add_u32(unsigned int* p, uint32_t v) {
-  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void st_relaxed_gpu_u32(unsigned int* p, uint32_t v) {
-  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
@@ -125,15 +111,6 @@ __device__ __forceinline__ void tma_load_4d(const CUtensorMap* m, uint64_t* bar,
       " [%0], [%1, {%3, %4, %5, %6}], [%2];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2),
       "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_5d(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1, int c2,
-                                            int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2),
-      "r"(c3), "r"(c4)
       : "memory");
 }
 __device__ __forceinline__ void tma_load_2d(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1) {
@@ -246,78 +223,6 @@ __host__ __device__ constexpr uint32_t make_idesc_f16(int m, int n, bool bf16, b
   return (1u << 4) | ((bf16 ? 1u : 0u) << 7) | ((bf16 ? 1u : 0u) << 10) | ((a_mn_major ? 1u : 0u) << 15) |
          ((b_mn_major ? 1u : 0u) << 16) | (static_cast<uint32_t>(n >> 3) << 17) |
          (static_cast<uint32_t>(m >> 4) << 24);
-}
-
-}  // namespace osvos
-
-// ===================== cluster / cta_group::2 (CTA pair) primitives =====================
-namespace osvos {
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of the same smem offset in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_shared(uint32_t local_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx_cluster(uint32_t bar_cluster_addr, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.release.cluster.shared::cluster.b64 _, [%0], %1;" ::"r"(bar_cluster_addr),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
-}
-// TMA loads whose completion is signalled on a barrier that may live in the peer CTA of the pair
-__device__ __forceinline__ void tma_load_4d_2sm(const CUtensorMap* m, uint32_t bar_cluster_addr, void* dst, int c0,
-                                                int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2),
-      "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_2sm(const CUtensorMap* m, uint32_t bar_cluster_addr, void* dst, int c0,
-                                                int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2cta(uint32_t* dst, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst)), "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2cta(uint32_t addr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
-}
-// D[tmem, 256 rows over the CTA pair] (+)= A * B; issued by one thread of the leader CTA.
-__device__ __forceinline__ void umma_f16_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                              uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive (once all prior MMAs of this thread completed) on the barrier at this smem offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(mask)
-      : "memory");
 }
 
 }  // namespace osvos

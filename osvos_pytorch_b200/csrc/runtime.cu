@@ -1,11 +1,14 @@
-// Library-level plumbing: version, thread-local error text, tensor-map encoding
+// Library-level plumbing: version, thread-local error text, environment switches, tensor-map encoding
 // through a run-time resolved driver entry point (no link-time libcuda
 // dependency, so the .so loads on a CPU-only box for the symbol tests).
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <map>
 #include <mutex>
+#include <optional>
+#include <string>
 
 #include "common.cuh"
 
@@ -70,6 +73,32 @@ int encode_tensor_map(CUtensorMap* map, CUtensorMapDataType dtype, int elem_byte
   return OSVOS_OK;
 }
 
+int encode_act_maps(CUtensorMap* hi, CUtensorMap* lo, const void* base_hi, const void* base_lo, int n, int h, int w, int c,
+                    int box_w, int box_h) {
+  const uint64_t dims[4] = {(uint64_t)c, (uint64_t)w, (uint64_t)h, (uint64_t)n};
+  const uint64_t strides[3] = {(uint64_t)c * 2, (uint64_t)w * c * 2, (uint64_t)h * w * c * 2};
+  const uint32_t box[4] = {64, (uint32_t)box_w, (uint32_t)box_h, 1};
+  const int rc = encode_tensor_map(hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, base_hi, dims, strides, box,
+                                   CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc) return rc;
+  return encode_tensor_map(lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, base_lo ? base_lo : base_hi, dims, strides, box,
+                           CU_TENSOR_MAP_SWIZZLE_128B);
+}
+
+int encode_weight_maps(CUtensorMap* hi, CUtensorMap* lo, const void* w_packed, int rows, int cin, int box_rows,
+                       int box_taps) {
+  const size_t plane = static_cast<size_t>(9) * rows * cin;  // elements
+  const uint64_t dims[3] = {(uint64_t)cin, (uint64_t)rows, 9};
+  const uint64_t strides[2] = {(uint64_t)cin * 2, (uint64_t)rows * cin * 2};
+  const uint32_t box[3] = {64, (uint32_t)box_rows, (uint32_t)box_taps};
+  const __nv_bfloat16* wp = static_cast<const __nv_bfloat16*>(w_packed);
+  const int rc = encode_tensor_map(hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp, dims, strides, box,
+                                   CU_TENSOR_MAP_SWIZZLE_128B);
+  if (rc) return rc;
+  return encode_tensor_map(lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp + plane, dims, strides, box,
+                           CU_TENSOR_MAP_SWIZZLE_128B);
+}
+
 int device_sm_count() {
   static int sms[64];
   int dev = 0;
@@ -82,18 +111,56 @@ int device_sm_count() {
   return sms[dev];
 }
 
-// Programmatic dependent launch: process default from OSVOS_PDL (read once), overridden per call sequence by
+// ---- environment switches -----------------------------------------------------------------------------------------
+// Every switch of the library is read here, by the same rule: once per process (the first read of a name is kept), or on
+// every call when OSVOS_ENV_RELOAD=1 was set at the first read - tests and scripts/ab_env.py flip switches inside one
+// process.  The defaults are the measured winners; the other values select A/B arms, cross-checks and diagnosis.
+//   OSVOS_HALO_LEAN=1      lean epilogue for plain forward halo launches (conv_common.cuh); 0: the general epilogue
+//   OSVOS_CONV_N256=1      256-wide halo tiles where they save a wave; 0: never
+//   OSVOS_SPLITACC128=1    N-concatenated split accumulator for 128-wide exact halo tiles; 0: three plain passes
+//   OSVOS_S1_SW64=1        fused stage-1 kernel with SWIZZLE_64B conv1_1 operands and a 5-stage weight ring;
+//                          0: 128-byte operand rows and 3 stages
+//   OSVOS_WGRAD_ROWS=1     weight gradient of Cin = Cout = 64 layers by tap rows; 0: by tap pairs
+//   OSVOS_WGRAD_SPLITS     unset: weight-gradient pixel splits chosen by cost; legacy: the first rule, ceil(2 SMs / tiles)
+//   OSVOS_SIDE_IMPL        unset: 16-output side convolutions on side_conv.cu; generic: the halo kernel's N = 16 tiles
+//   OSVOS_FIRST_IMPL       unset: conv1_1 on the tensor cores (conv_first_tc.cu); simt: the CUDA-core kernel
+//   OSVOS_ABLATE=0         timing ablation bit mask of the conv kernels (ConvParams::ablate; results are garbage)
+//   OSVOS_PDL=0            programmatic dependent launch; osvos_set_pdl() overrides it
+// (The engine's own switches - OSVOS_FUSE_STAGE1, OSVOS_FOLD_SIDE, ... - are read by engine.py on every call.)
+static const char* env_str(const char* name) {
+  static const bool reload = [] {
+    const char* e = getenv("OSVOS_ENV_RELOAD");
+    return e != nullptr && atoi(e) != 0;
+  }();
+  if (reload) return getenv(name);
+  static std::mutex mu;
+  static std::map<std::string, std::optional<std::string>> first_read;
+  std::lock_guard<std::mutex> lock(mu);
+  auto it = first_read.find(name);
+  if (it == first_read.end()) {
+    const char* e = getenv(name);
+    it = first_read.emplace(name, e ? std::optional<std::string>(e) : std::nullopt).first;
+  }
+  return it->second ? it->second->c_str() : nullptr;
+}
+
+int env_int(const char* name, int dflt) {
+  const char* e = env_str(name);
+  return e == nullptr ? dflt : atoi(e);
+}
+
+bool env_is(const char* name, const char* value) {
+  const char* e = env_str(name);
+  return e != nullptr && strcmp(e, value) == 0;
+}
+
+// Programmatic dependent launch: process default from OSVOS_PDL, overridden per call sequence by
 // osvos_set_pdl() - the engine switches it on around the inference pass (measured +1.4 % there, -1.7 % on the fwd+bwd
 // graph: profiles/r01f_pdl_ab.txt).  A captured graph keeps the attribute its launches were captured with.
 static int g_pdl_override = -1;   // -1: environment default
 bool pdl_enabled() {
   if (g_pdl_override >= 0) return g_pdl_override == 1;
-  static int state = -1;
-  if (state < 0) {
-    const char* e = getenv("OSVOS_PDL");
-    state = (e != nullptr && atoi(e) != 0) ? 1 : 0;
-  }
-  return state == 1;
+  return env_int("OSVOS_PDL", 0) != 0;
 }
 
 }  // namespace osvos

@@ -375,8 +375,7 @@ extern "C" int osvos_side_folded_wgrad_multi(const osvos_side_wgrad_item* items,
     p.sc[k].blocks = static_cast<int>(b * slabs);
     begin += p.sc[k].blocks;
   }
-  static uint64_t attr_done = 0;
-  OSVOS_CHECK_CUDA(ensure_dynamic_smem(side_folded_wgrad_kernel, kSwSmemBytes, &attr_done));
+  OSVOS_CHECK_CUDA(ensure_dynamic_smem<side_folded_wgrad_kernel>(kSwSmemBytes));
   OSVOS_CHECK_CUDA(launch_pdl(side_folded_wgrad_kernel, dim3(begin), dim3(kSwKernelThreads), kSwSmemBytes,
                               static_cast<cudaStream_t>(stream_), maps, p));
   return OSVOS_OK;
@@ -421,9 +420,8 @@ extern "C" int osvos_side_grads_finish(const osvos_side_grads_item* items, int c
   for (int i = 0; i < count; ++i) cmax = items[i].c > cmax ? items[i].c : cmax;
   OSVOS_CHECK_ARG(cmax <= 2048);
   const size_t smem = (static_cast<size_t>(18) * (cmax + 1) + 2) * sizeof(float);
-  static uint64_t attr_done = 0;
   if (smem > 48 * 1024)
-    OSVOS_CHECK_CUDA(ensure_dynamic_smem(side_grads_finish_kernel, (18 * 2049 + 2) * static_cast<int>(sizeof(float)), &attr_done));
+    OSVOS_CHECK_CUDA(ensure_dynamic_smem<side_grads_finish_kernel>((18 * 2049 + 2) * static_cast<int>(sizeof(float))));
   OSVOS_CHECK_CUDA(launch_pdl(side_grads_finish_kernel, dim3(16 * count), dim3(kFinThreads), smem, static_cast<cudaStream_t>(stream_), t));
   return OSVOS_OK;
 }

@@ -355,30 +355,11 @@ static int launch_side(const osvos_conv3x3_args* const* args, int count, cudaStr
     L.relu = (a->flags & OSVOS_FLAG_RELU) ? 1 : 0;
     L.tile_begin = total;
     total += L.tiles_x * L.tiles_y * a->n;
-    {
-      const uint64_t dims[4] = {(uint64_t)a->cin, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-      const uint64_t strides[3] = {(uint64_t)a->cin * 2, (uint64_t)a->w * a->cin * 2, (uint64_t)a->h * a->w * a->cin * 2};
-      const uint32_t box[4] = {64, kSideHaloW, kSideHaloH, 1};
-      int rc = encode_tensor_map(&maps.x_hi[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, a->x_hi, dims, strides, box,
-                                 CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-      rc = encode_tensor_map(&maps.x_lo[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, PLANES == 2 ? a->x_lo : a->x_hi, dims,
-                             strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-    }
-    {
-      const size_t plane = static_cast<size_t>(9) * NCO * a->cin;
-      const uint64_t dims[3] = {(uint64_t)a->cin, NCO, 9};
-      const uint64_t strides[2] = {(uint64_t)a->cin * 2, (uint64_t)NCO * a->cin * 2};
-      const uint32_t box[3] = {64, NCO, 9};
-      const __nv_bfloat16* wp = static_cast<const __nv_bfloat16*>(a->w_packed);
-      int rc = encode_tensor_map(&maps.w_hi[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp, dims, strides, box,
-                                 CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-      rc = encode_tensor_map(&maps.w_lo[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 3, wp + plane, dims, strides, box,
-                             CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-    }
+    int rc = encode_act_maps(&maps.x_hi[k], &maps.x_lo[k], a->x_hi, PLANES == 2 ? a->x_lo : nullptr, a->n, a->h, a->w,
+                             a->cin, kSideHaloW, kSideHaloH);
+    if (rc) return rc;
+    rc = encode_weight_maps(&maps.w_hi[k], &maps.w_lo[k], a->w_packed, NCO, a->cin, NCO, 9);   // all nine taps
+    if (rc) return rc;
   }
   for (int k = count; k < kSideMaxScales; ++k) {   // unused slots: valid descriptors (never dereferenced)
     maps.x_hi[k] = maps.x_hi[0];
@@ -387,12 +368,8 @@ static int launch_side(const osvos_conv3x3_args* const* args, int count, cudaStr
     maps.w_lo[k] = maps.w_lo[0];
   }
   p.total_tiles = total;
-  auto kern = side_conv_kernel<PLANES, NCO>;
-  static uint64_t attr_done = 0;   // per instantiation: bit d = device d has the shared-memory opt-in
-  OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, Cfg::kSmem, &attr_done));
-  const int sms = device_sm_count();
-  const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-  OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kSideThreads), Cfg::kSmem, stream, maps, p));
+  OSVOS_CHECK_CUDA((launch_persistent<side_conv_kernel<PLANES, NCO>>(p.total_tiles, kSideThreads, Cfg::kSmem, stream, maps,
+                                                                     p)));
   return OSVOS_OK;
 }
 

@@ -17,11 +17,11 @@
 // Work item = (m block of 128, n block, tap, pixel-range split); the fp32 TMEM
 // accumulator is flushed with vector atomics (red.global.add.v4.f32) into the
 // zero-initialised workspace, which a small kernel then transposes into the
-// OIHW gradient.  Same warp roles / mbarrier pipeline as conv3x3_tc.cu.
+// OIHW gradient.  Warps 0 and 6 are the TMA producers of P and Q, warp 1 the MMA
+// issuer, warps 2-5 the epilogue; mbarrier rings as in conv3x3_halo.cu.
 //
 // Replaces autograd's weight gradient of nn.Conv2d(k=3, p=1)
 // (reference networks/vgg_osvos.py:41,142; backward triggered at train_online.py:141).
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -381,22 +381,12 @@ wgrad_finish_multi_kernel(const __grid_constant__ FinishTable t) {
   }
 }
 
-// Environment switches of launch_wgrad (A/B; read once).
+// The switches of launch_wgrad: OSVOS_WGRAD_ROWS, OSVOS_WGRAD_SPLITS (runtime.cu).
 struct WgradSwitches {
-  bool rows;          // OSVOS_WGRAD_ROWS     (default 1): tap rows for Cin = Cout = 64; 0: tap pairs instead
-  bool legacy_split;  // OSVOS_WGRAD_SPLITS=legacy: the first split rule
+  bool rows, legacy_split;
 };
 static WgradSwitches wgrad_switches() {
-  static int rows_on = -1, split_rule = -1;
-  if (rows_on < 0) {
-    const char* e = getenv("OSVOS_WGRAD_ROWS");
-    rows_on = (e == nullptr || atoi(e) != 0) ? 1 : 0;
-  }
-  if (split_rule < 0) {
-    const char* e = getenv("OSVOS_WGRAD_SPLITS");
-    split_rule = (e != nullptr && strcmp(e, "legacy") == 0) ? 1 : 0;
-  }
-  return WgradSwitches{rows_on == 1, split_rule == 1};
+  return WgradSwitches{env_int("OSVOS_WGRAD_ROWS", 1) != 0, env_is("OSVOS_WGRAD_SPLITS", "legacy")};
 }
 
 // The work decomposition of one launch: every WgradParams field that is not a pointer or an image dimension, and the
@@ -458,51 +448,38 @@ static int plan_wgrad(const osvos_wgrad_args* a, int block_n, int sms, const Wgr
   p.patches_per_split = (p.patches_total + splits - 1) / splits;
   p.splits = (p.patches_total + p.patches_per_split - 1) / p.patches_per_split;
   p.total_items = tiles * p.splits;
-  grid = p.total_items < sms ? p.total_items : sms;
+  grid = persistent_grid(p.total_items, sms);
   return OSVOS_OK;
 }
 
 template <int BLOCK_N, int PLANES>
 static int launch_wgrad(const osvos_wgrad_args* a, cudaStream_t stream) {
   using Cfg = WgCfg<BLOCK_N, PLANES>;
-  // operand roles
-  const void* p_hi = a->dz_hi;
-  const void* p_lo = a->dz_lo;
-  const void* q_hi = a->x_hi;
-  const void* q_lo = a->x_lo;
-  const int cp = a->dz_channels;   // channels of the P tensor
-  const int cq = a->cin;           // channels of the Q tensor
-
   WgradParams p;
   int grid = 0;
-  const int rc_plan = plan_wgrad(a, BLOCK_N, device_sm_count(), wgrad_switches(), p, grid);
-  if (rc_plan) return rc_plan;
+  int rc = plan_wgrad(a, BLOCK_N, device_sm_count(), wgrad_switches(), p, grid);
+  if (rc) return rc;
   p.ws = a->workspace;
 
+  // operands: P = dz (dz_channels), Q = the layer's input x (cin)
   CUtensorMap mp_hi, mp_lo, mq_hi, mq_lo;
-  auto enc = [&](CUtensorMap* m, const void* base, int c) {
-    const uint64_t dims[4] = {(uint64_t)c, (uint64_t)a->w, (uint64_t)a->h, (uint64_t)a->n};
-    const uint64_t strides[3] = {(uint64_t)c * 2, (uint64_t)a->w * c * 2, (uint64_t)a->h * a->w * c * 2};
-    const uint32_t box[4] = {64, kWgPatchW, kWgPatchH, 1};
-    return encode_tensor_map(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 4, base, dims, strides, box,
-                             CU_TENSOR_MAP_SWIZZLE_128B);
-  };
-  int rc;
-  if ((rc = enc(&mp_hi, p_hi, cp))) return rc;
-  if ((rc = enc(&mp_lo, PLANES == 2 ? p_lo : p_hi, cp))) return rc;
-  if ((rc = enc(&mq_hi, q_hi, cq))) return rc;
-  if ((rc = enc(&mq_lo, PLANES == 2 ? q_lo : q_hi, cq))) return rc;
+  rc = encode_act_maps(&mp_hi, &mp_lo, a->dz_hi, PLANES == 2 ? a->dz_lo : nullptr, a->n, a->h, a->w, a->dz_channels,
+                       kWgPatchW, kWgPatchH);
+  if (rc) return rc;
+  rc = encode_act_maps(&mq_hi, &mq_lo, a->x_hi, PLANES == 2 ? a->x_lo : nullptr, a->n, a->h, a->w, a->cin, kWgPatchW,
+                       kWgPatchH);
+  if (rc) return rc;
 
-  const bool deferred = (a->flags & OSVOS_FLAG_DEFER_FINISH) != 0;
-  const size_t ws_bytes = static_cast<size_t>(9) * p.m_total * p.n_total * sizeof(float);
-  if (!deferred) OSVOS_CHECK_CUDA(cudaMemsetAsync(a->workspace, 0, ws_bytes, stream));
-  auto kern = wgrad_tc_kernel<BLOCK_N, PLANES>;
-  static uint64_t attr_done = 0;   // per instantiation: bit d = device d has the shared-memory opt-in
-  OSVOS_CHECK_CUDA(ensure_dynamic_smem(kern, Cfg::kSmemBytes, &attr_done));
-  if (deferred) {   // (otherwise the memset above is this kernel's stream predecessor: plain launch)
-    OSVOS_CHECK_CUDA(launch_pdl(kern, dim3(grid), dim3(kWgThreads), Cfg::kSmemBytes, stream, mp_hi, mp_lo, mq_hi, mq_lo, p));
+  constexpr auto kern = wgrad_tc_kernel<BLOCK_N, PLANES>;
+  if (a->flags & OSVOS_FLAG_DEFER_FINISH) {
+    OSVOS_CHECK_CUDA((launch_persistent<kern>(p.total_items, kWgThreads, Cfg::kSmemBytes, stream, mp_hi, mp_lo, mq_hi,
+                                              mq_lo, p)));
     return OSVOS_OK;
   }
+  // immediate form: the memset is this kernel's stream predecessor, so a plain launch
+  const size_t ws_bytes = static_cast<size_t>(9) * p.m_total * p.n_total * sizeof(float);
+  OSVOS_CHECK_CUDA(cudaMemsetAsync(a->workspace, 0, ws_bytes, stream));
+  OSVOS_CHECK_CUDA(ensure_dynamic_smem<kern>(Cfg::kSmemBytes));
   kern<<<grid, kWgThreads, Cfg::kSmemBytes, stream>>>(mp_hi, mp_lo, mq_hi, mq_lo, p);
   OSVOS_CHECK_CUDA(cudaGetLastError());
   const int total = a->cout * a->cin * 9;

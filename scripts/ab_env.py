@@ -7,6 +7,7 @@ four rotating frames (CUDA events), and the five output maps are compared with t
 """
 import os
 import sys
+os.environ.setdefault("OSVOS_ENV_RELOAD", "1")   # the library re-reads its switches on every launch (csrc/runtime.cu)
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 torch.set_grad_enabled(False)
